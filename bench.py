@@ -16,6 +16,7 @@ Workloads (--workload; the default is the one BASELINE.json's metric is quoted o
   dpr              configs[4]: DPR BiEncoder (BERT-base, CLS, no head), L=256, 21,015,324 x 768 un-normalised rows, top-100
 
   python bench.py --gpus 1 --steps 5 --warmup 3
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # + the last timed step's outputs as DIR/<name>.npy
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...     # the reference's CPU arithmetic on the host cores (see run_reference)
@@ -347,6 +348,21 @@ def build_model(wl, dev, encoder_operand):
     return model.to(dev).eval()
 
 
+DUMP_MAX_ROWS = 4096
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output as out_dir/<name>.npy: float32, labels as float64 (exact below 2**53).  An output of more than
+    DUMP_MAX_ROWS rows keeps the rows np.random.default_rng(0).choice(n, DUMP_MAX_ROWS, replace=False), sorted: the same
+    rows in every run, so that two builds can be compared output for output (at most ~32 MB in all)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in outputs.items():
+        x = x.cpu().numpy() if torch.is_tensor(x) else np.asarray(x)
+        if x.shape[0] > DUMP_MAX_ROWS:
+            x = x[np.sort(np.random.default_rng(0).choice(x.shape[0], DUMP_MAX_ROWS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), x.astype(np.float64 if x.dtype.kind in "iu" else np.float32))
+
+
 def run_b200(args, wl):
     import torch.distributed as dist
     from ance_b200 import _lib
@@ -402,6 +418,7 @@ def run_b200(args, wl):
             model.encode_lens(ids, lens, out=step_rows)
 
     pending = []      # N > 1: the previous slice's search, issued but not yet merged / gathered
+    last = {}         # what the latest step computed (--dump-outputs): its queries and, once merged, their top-k labels
 
     def step_value():
         step_index.reset()
@@ -410,18 +427,24 @@ def run_b200(args, wl):
         step_index.prepare()               # column mean + centred 16-bit operands + norm statistics of the added rows
         q = model.query_emb(q_ids_d, q_ids_d != 0) if mask_form else model.encode_lens(q_ids_d, q_len_d)
         if world == 1:
-            return sharded_search(local_search, n_local, q.contiguous(), k, row_offset=row_offset)   # numpy labels
+            last["query_emb"] = q
+            last["topk_labels"] = sharded_search(local_search, n_local, q.contiguous(), k, row_offset=row_offset)
+            return last["topk_labels"]     # numpy labels
         q_all = torch.empty((qb * world, DIM), dtype=torch.float32, device=dev)
         dist.all_gather_into_tensor(q_all, q.contiguous())
+        last["query_emb"] = q_all
         # As in the driver's block loop, the host merge of this slice's lists overlaps the device work that follows: the
         # search is issued here and finished (merge waited for, labels gathered on rank 0) after the NEXT slice has been
         # enqueued; `drain()` finishes the last one inside the timed region.
         pending.append(sharded_search_start(local_search, n_local, q_all, k, row_offset=row_offset))
-        return pending.pop(0).finish() if len(pending) > 1 else None
+        if len(pending) > 1:
+            last["topk_labels"] = pending.pop(0).finish()
+            return last["topk_labels"]
+        return None
 
     def drain():
         while pending:
-            pending.pop(0).finish()
+            last["topk_labels"] = pending.pop(0).finish()
 
     def step_e2e():
         """The calls a user of the reference makes (run_ann_data_gen.py:172-180,269-303), host buffers in, numpy out:
@@ -479,6 +502,9 @@ def run_b200(args, wl):
     prof = _lib.profile_read(reset=True)
     _lib.profile_enable(False)
     launches = _lib.load().ance_launch_count() - launches0
+    if args.dump_outputs and rank == 0:    # before the e2e pass below writes its own passages into step_rows
+        dump_outputs(args.dump_outputs, {"passage_emb": step_rows, "query_emb": last["query_emb"],
+                                         "topk_labels": last["topk_labels"]})
     st = index.stats()
     step_e2e()
     ms_e2e = timed(step_e2e, max(2, args.steps // 2), wall=True)
@@ -615,7 +641,12 @@ def main():
     ap.add_argument("--search_operand", default="auto", choices=["auto", "fp16", "bf16"])
     ap.add_argument("--encoder_operand", default="fp16", choices=["fp16", "bf16"])
     ap.add_argument("--no_cpu_baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (passage and query embeddings, top-k "
+                         "labels) as DIR/<name>.npy; the inputs are seeded, so runs with the same arguments compare")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     wl = WORKLOADS[args.workload]
     # defaults: marco_psg 64 encoder passes of 592 x 128 tokens + 2 of 1184 x 64 (16:1, the refresh's own 17.6:1);
     # marco_doc_maxp 64 passes of 148 x 512 (2,368 documents) + 296 queries (8:1; real 8.75:1); dpr 64 passes of 296 x 256

@@ -32,3 +32,31 @@ def test_reference_arm_json_line():
 
 def test_reference_arm_other_ranks_are_silent():
     assert _run({"RANK": "1", "WORLD_SIZE": "2"}) == []
+
+
+def test_dump_outputs_is_a_fixed_sample_in_float(tmp_path):
+    """--dump-outputs: outputs land as <name>.npy in float32 / float64 (labels exact), larger ones as the same seeded
+    sample of rows in every run, all of it within 64 MB at the default workload's sizes."""
+    import numpy as np
+    import torch
+
+    import bench
+    rng = np.random.default_rng(1)
+    outputs = {"passage_emb": torch.from_numpy(rng.standard_normal((37888, 768), dtype=np.float32)),
+               "query_emb": rng.standard_normal((2368, 768), dtype=np.float32),
+               "topk_labels": rng.integers(0, 8841823, size=(2368, 200))}
+    bench.dump_outputs(str(tmp_path / "a"), outputs)
+    bench.dump_outputs(str(tmp_path / "b"), outputs)
+    total = 0
+    for name in outputs:
+        a, b = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert np.array_equal(a, b) and a.shape[0] == min(bench.DUMP_MAX_ROWS, len(outputs[name]))
+        total += a.nbytes
+    assert np.load(tmp_path / "a" / "query_emb.npy").dtype == np.float32
+    labels = np.load(tmp_path / "a" / "topk_labels.npy")
+    assert labels.dtype == np.float64 and np.array_equal(labels, outputs["topk_labels"])
+    P, rows = outputs["passage_emb"].numpy(), np.load(tmp_path / "a" / "passage_emb.npy")
+    idx = np.searchsorted(np.sort(P[:, 0]), rows[:, 0])
+    idx = np.argsort(P[:, 0])[idx]                      # the input row each dumped row came from
+    assert np.array_equal(P[idx], rows) and (np.diff(idx) > 0).all()
+    assert total <= 64 << 20
