@@ -16,7 +16,7 @@
 //   4. tier 2, for the queries step 3 could not certify: the SAME coarse kernel once more over those queries only,
 //      started from a per-query threshold t(q) = s_k - eps(q) (s_k = k-th exact score found so far, a lower bound of
 //      the true one).  Every row that can still belong to the top-k has coarse score > t(q), so unless more than
-//      ~2000 rows per split sit within eps of the boundary nothing is dropped and the result is certified BY
+//      ~2000 rows per split (~4000 / ~8000 above k = 512 / 1024) sit within eps of the boundary nothing is dropped and the result is certified BY
 //      CONSTRUCTION: a failed certificate costs one more coarse pass over the failed queries, not a brute force.
 //   5. exact_* kernels : what is left (thousands of near-ties at the boundary: duplicated rows, adversarial data) is
 //      recomputed by brute force in exact arithmetic.  Also the validation path (ance_index_search_exact).
@@ -33,6 +33,11 @@
 namespace {
 
 using namespace tc05;
+
+// Largest k ance_index_search / ance_index_search_exact accept (faiss's GPU flat index has the same limit).
+constexpr int kMaxK = 2048;
+// Largest k' (candidates kept per split): the default for bf16 operands at k = kMaxK, 2 k + 32.
+constexpr int kMaxKprime = 2 * kMaxK + 32;
 
 // ------------------------------------------------------------------------------------------------
 // order-preserving float <-> uint32 (larger float -> larger key)
@@ -166,8 +171,12 @@ struct EpTopK {
   static constexpr uint64_t kHintB = tc05::kEvictNormal;  // corpus rows: every concurrently sweeping CTA pair re-reads
                                                           // the same tile from L2 (EVICT_FIRST made each pair go to
                                                           // HBM: 788 GB of DRAM reads for 13.6 GB of operands, ncu r01)
-  static constexpr int kSlots = CAP / 32;
-  static constexpr int kSmemBytes = 0;
+  // CAP <= 2048: the reservoir is selected in registers (kSlots keys and ids per lane).  Larger reservoirs (k > 512) do
+  // not fit there: compact_wide selects them where they are, in global memory (L2), with a 256-bin histogram per
+  // epilogue warp in shared memory.
+  static constexpr bool kWide = CAP > 2048;
+  static constexpr int kEpiWarps = 4;
+  static constexpr int kSmemBytes = kWide ? kEpiWarps * 256 * 4 : 0;
   struct Params {
     float* scratch_sc;  // [gridDim.x * 128 * CAP] reservoir scores
     int* scratch_id;    // [gridDim.x * 128 * CAP] reservoir rows
@@ -199,6 +208,7 @@ struct EpTopK {
   // (radix select on the order-preserving key, stable compaction: among equal scores the earlier
   // = lower row wins).  Afterwards src.cnt = kprime and src.thr = kprime-th best coarse score.
   __device__ __forceinline__ void compact(int kprime, int src, int lane) {
+    constexpr int kSlots = CAP / 32;
     const int n = __shfl_sync(0xffffffffu, cnt, src);
     float* s_sc = shfl_ptr(sc, src);
     int* s_id = shfl_ptr(id, src);
@@ -248,6 +258,103 @@ struct EpTopK {
     }
   }
 
+  // Same selection and the same result as compact() for a reservoir too large for registers: four passes of an
+  // 8-bit-digit radix select (most significant digit first) over the reservoir in place, each counting the entries
+  // that match the digits chosen so far into the warp's shared histogram, then the same stable in-place compaction.
+  // Every dropped entry has key < T, or key == T behind the `remaining` kept ones: coarse score <= thr, as the
+  // certificate requires.
+  __device__ __forceinline__ void compact_wide(int kprime, int src, int lane, uint32_t* hist) {
+    const int n = __shfl_sync(0xffffffffu, cnt, src);
+    float* s_sc = shfl_ptr(sc, src);
+    int* s_id = shfl_ptr(id, src);
+    uint32_t prefix = 0, pmask = 0;
+    int remaining = kprime;   // n > kprime: entries matching the prefix always number >= remaining
+#pragma unroll 1
+    for (int shift = 24; shift >= 0; shift -= 8) {
+      for (int b = lane; b < 256; b += 32) hist[b] = 0u;
+      __syncwarp();
+      for (int i0 = 0; i0 < n; i0 += 32) {
+        // lanes whose entries share a digit add once for all of them: in the first passes most entries fall in a few
+        // bins, and 32 atomics on one shared-memory address serialise
+        const int i = i0 + lane;
+        uint32_t bin = 256u;   // no entry, or one that does not match the digits chosen so far
+        if (i < n) {
+          const uint32_t key = f2ord(s_sc[i]);
+          if ((key & pmask) == prefix) bin = (key >> shift) & 255u;
+        }
+        const unsigned peers = __match_any_sync(0xffffffffu, bin);
+        if (bin < 256u && lane == __ffs(peers) - 1) atomicAdd(&hist[bin], static_cast<uint32_t>(__popc(peers)));
+      }
+      __syncwarp();
+      // lane l owns digits 8l .. 8l+7; `above` = entries whose digit belongs to a higher lane
+      int c[8], tot = 0;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        c[j] = static_cast<int>(hist[lane * 8 + j]);
+        tot += c[j];
+      }
+      int suf = tot;
+#pragma unroll
+      for (int s = 1; s < 32; s <<= 1) {
+        const int v = __shfl_down_sync(0xffffffffu, suf, s);
+        if (lane + s < 32) suf += v;
+      }
+      const int above = suf - tot;
+      const bool mine = above < remaining && remaining <= suf;   // exactly one lane
+      int digit = 0, rem = 0;
+      if (mine) {
+        int acc = above;
+#pragma unroll
+        for (int j = 7; j >= 0; --j) {
+          if (acc + c[j] >= remaining) {
+            digit = lane * 8 + j;
+            rem = remaining - acc;
+            break;
+          }
+          acc += c[j];
+        }
+      }
+      const int owner = __ffs(__ballot_sync(0xffffffffu, mine)) - 1;
+      digit = __shfl_sync(0xffffffffu, digit, owner);
+      remaining = __shfl_sync(0xffffffffu, rem, owner);
+      prefix |= static_cast<uint32_t>(digit) << shift;
+      pmask |= 255u << shift;
+    }
+    const uint32_t T = prefix;
+    const unsigned lt = (1u << lane) - 1u;
+    int base = 0, eq_seen = 0;
+#pragma unroll 1
+    for (int i0 = 0; i0 < n; i0 += 32) {
+      const int i = i0 + lane;
+      const bool v = i < n;
+      const float s = v ? s_sc[i] : 0.f;
+      const int rid = v ? s_id[i] : -1;
+      const uint32_t key = f2ord(s);
+      const bool gt = v && key > T, eq = v && key == T;
+      const unsigned eqm = __ballot_sync(0xffffffffu, eq);
+      const bool keep = gt || (eq && (eq_seen + __popc(eqm & lt)) < remaining);
+      const unsigned km = __ballot_sync(0xffffffffu, keep);
+      __syncwarp();   // every lane has read its entry of this chunk before any lane overwrites one (pos <= i0 + 31)
+      if (keep) {
+        const int pos = base + __popc(km & lt);
+        s_sc[pos] = s;
+        s_id[pos] = rid;
+      }
+      base += __popc(km);
+      eq_seen += __popc(eqm);
+    }
+    __syncwarp();
+    if (lane == src) {
+      cnt = kprime;
+      thr = ord2f(T);
+    }
+  }
+
+  __device__ __forceinline__ void compact_any(int kprime, int src, const gemm::EpiCtx& cx) {
+    if constexpr (kWide) compact_wide(kprime, src, cx.lane, reinterpret_cast<uint32_t*>(cx.ep_smem) + cx.epi_warp * 256);
+    else compact(kprime, src, cx.lane);
+  }
+
   __device__ __forceinline__ void tile(const Params& p, const gemm::WorkShape&, const gemm::EpiCtx& cx,
                                        uint32_t tacc, int nb) {
 #pragma unroll 1
@@ -275,7 +382,7 @@ struct EpTopK {
       while (need) {
         const int src = __ffs(need) - 1;
         need &= need - 1;
-        compact(p.kprime, src, cx.lane);
+        compact_any(p.kprime, src, cx);
       }
     }
   }
@@ -288,7 +395,7 @@ struct EpTopK {
     while (need) {
       const int src = __ffs(need) - 1;
       need &= need - 1;
-      compact(p.kprime, src, cx.lane);
+      compact_any(p.kprime, src, cx);
     }
     for (int l = 0; l < 32; ++l) {
       const int row = cx.row0 + cx.quad * 32 + l;
@@ -529,8 +636,17 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
 // 4. exact brute force (fallback for uncertified queries, and the validation path)
 // ------------------------------------------------------------------------------------------------
 constexpr int kExQB = 4;       // queries per block
-constexpr int kExBuf = 1024;   // reservoir keys per query
 constexpr int kExRound = 16;   // rows per warp between reservoir checks
+constexpr int kExWarps = 8;    // 256 threads
+// reservoir keys per query (kExBuf, a template argument): a compacted reservoir holds k keys and takes up to
+// kExWarps * kExRound more before the next check, so at least k + kExWarps * kExRound; and at least 2 k, so that a
+// compaction (a block-wide sort) is paid for by about k new keys, not by one round's.  A power of two: 1024 for every
+// k <= 512, 2048 up to k = 1024, 4096 up to k = 2048.
+__host__ __device__ constexpr int exact_buf_keys(int k) {
+  int b = 1024;
+  while (b < k + kExWarps * kExRound || b < 2 * k) b <<= 1;
+  return b;
+}
 
 struct ExactParams {
   const float* Q;
@@ -541,11 +657,12 @@ struct ExactParams {
   int q_base;
   const int* nq_dev;     // number of queries on the device (null = use nq)
   int nq;
-  int k;                 // <= 512
+  int k;                 // <= kMaxK
   int n_chunks;
   uint64_t* chunk_keys;  // [nq_cap * n_chunks * k]
 };
 
+template <int kExBuf>
 __global__ void __launch_bounds__(256) exact_chunk_kernel(const ExactParams p) {
   extern __shared__ __align__(16) uint8_t ex_smem[];
   uint64_t* buf = reinterpret_cast<uint64_t*>(ex_smem);              // [kExQB][kExBuf]
@@ -631,6 +748,7 @@ __global__ void __launch_bounds__(256) exact_chunk_kernel(const ExactParams p) {
 }
 
 constexpr int kMergeBuf = 4096;
+static_assert(kMergeBuf >= 2 * kMaxK, "exact_merge_kernel takes kMergeBuf - k new keys per round");
 
 __global__ void __launch_bounds__(256) exact_merge_kernel(const ExactParams p, float* D, int64_t* I, int out_k,
                                                           int64_t row_offset) {
@@ -754,6 +872,18 @@ int check_handle_device(const ance_index* ix, const char* who) {
   return ANCE_OK;
 }
 
+// Reservoir entries per query row of the coarse epilogue for a given k': room for about k' more survivors between two
+// compactions.  k <= 512 only ever uses 1024 and 2048 (k' <= 992).
+int reservoir_cap(int kprime) { return kprime <= 512 ? 1024 : kprime <= 1024 ? 2048 : kprime <= 2048 ? 4096 : 8192; }
+
+// Candidates per query above k = 512, all splits together: the rescore's shared-memory sort, 16384 keys = 128 KB.
+constexpr int kMaxCands = 16384;
+static_assert(kMaxKprime <= kMaxCands, "one split's candidates must fit the rescore's sort");
+
+// k' of tier 2 (its reservoir is compacted only when it overflows, dropping candidates): half a reservoir less one
+// compaction check — CAP 2048 for k <= 512 (as it always was), 4096 up to k = 1024, 8192 up to kMaxK.
+int tier2_kprime(int k) { return k <= 512 ? 992 : k <= 1024 ? 2016 : 4064; }
+
 template <int BN, int STAGES, int CG, int CAP, uint32_t FMT>
 int launch_coarse(ance_index* ix, const uint16_t* Q16, int64_t nq, int kprime, int out_cap, const float* thr_init,
                   int n_splits_req, int* n_splits_out, cudaStream_t st) {
@@ -771,11 +901,14 @@ int launch_coarse(ance_index* ix, const uint16_t* Q16, int64_t nq, int kprime, i
     return ANCE_ERR_CUDA;
   }
   const int ctas = (ix->max_ctas > 0 ? ix->max_ctas : gemm::sm_count());
+  // one reservoir of max(CAP, 2048) entries per (CTA, query row): the large-k reservoirs (CAP 8192: 1.2 GB on 148 SMs)
+  // are allocated only when a large k is searched
+  const size_t res = static_cast<size_t>(ctas) * gemm::BM * std::max(CAP, 2048);
   size_t se = ix->scratch_elems;
-  int rc = ensure(&ix->scratch_sc, &se, static_cast<size_t>(ctas) * gemm::BM * 2048);
+  int rc = ensure(&ix->scratch_sc, &se, res);
   if (rc) return rc;
   se = ix->scratch_elems;
-  rc = ensure(&ix->scratch_id, &se, static_cast<size_t>(ctas) * gemm::BM * 2048);
+  rc = ensure(&ix->scratch_id, &se, res);
   if (rc) return rc;
   ix->scratch_elems = se;
   const size_t slots = static_cast<size_t>(nq) * ws.n_splits;
@@ -831,26 +964,34 @@ int run_exact(ance_index* ix, const float* Q, const int* qlist, int nq, int k, f
   ep.n_rows = ix->n;
   ep.nq_dev = nullptr;
   ep.k = static_cast<int>(std::min<int64_t>(k, std::max<int64_t>(ix->n, 1)));
-  ep.k = std::min(ep.k, 512);
+  ep.k = std::min(ep.k, kMaxK);
   const int sms = gemm::sm_count();
   int n_chunks = static_cast<int>(std::min<int64_t>(2 * sms, (ix->n + 4095) / 4096));
   if (n_chunks < 1) n_chunks = 1;
   ep.n_chunks = n_chunks;
-  const int batch = std::min(nq, kExactBatch);
+  // the chunk_keys scratch grows with batch * n_chunks * k: above k = 512 the batch shrinks so that it stays the size
+  // it has at k = 512 (1.2 GB with 296 chunks)
+  const int per_pass = (ep.k <= 512) ? kExactBatch : std::max(1, kExactBatch * 512 / ep.k);
+  const int batch = std::min(nq, per_pass);
   int rc = ensure(&ix->chunk_keys, &ix->chunk_keys_elems, static_cast<size_t>(batch) * n_chunks * ep.k);
   if (rc) return rc;
   ep.chunk_keys = ix->chunk_keys;
-  const size_t smem = static_cast<size_t>(kExQB) * kExBuf * 8 + static_cast<size_t>(kExQB) * ix->dim * 4;
+  const int buf = exact_buf_keys(ep.k);
+  const size_t smem = static_cast<size_t>(kExQB) * buf * 8 + static_cast<size_t>(kExQB) * ix->dim * 4;
+  void (*chunk)(const ExactParams) = (buf == 1024) ? exact_chunk_kernel<1024>
+                                   : (buf == 2048) ? exact_chunk_kernel<2048> : exact_chunk_kernel<4096>;
+  static_assert(exact_buf_keys(kMaxK) <= 4096, "exact_chunk_kernel instantiations");
   // per device and cheap: set on every call rather than behind a process-wide flag
-  ANCE_CUDA(cudaFuncSetAttribute(exact_chunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-  for (int b0 = 0; b0 < nq; b0 += kExactBatch) {
-    const int nb = std::min(kExactBatch, nq - b0);
+  ANCE_CUDA(cudaFuncSetAttribute(chunk, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 static_cast<int>(std::max<size_t>(100 * 1024, smem))));
+  for (int b0 = 0; b0 < nq; b0 += per_pass) {
+    const int nb = std::min(per_pass, nq - b0);
     ep.qlist = qlist ? qlist + b0 : nullptr;
     ep.q_base = b0;
     ep.nq = nb;
     const int gy = std::max(1, std::min((nb + kExQB - 1) / kExQB, 128));
     ance::ProfScope ps(ance::kClsExact, st);
-    exact_chunk_kernel<<<dim3(n_chunks, gy), 256, smem, st>>>(ep);
+    chunk<<<dim3(n_chunks, gy), 256, smem, st>>>(ep);
     ANCE_CUDA(cudaGetLastError());
     exact_merge_kernel<<<std::max(1, std::min(nb, 4 * sms)), 256, 0, st>>>(ep, D, I, k, row_offset);
     ANCE_CUDA(cudaGetLastError());
@@ -869,9 +1010,12 @@ int coarse_rescore_pass(ance_index* ix, const uint16_t* Q16, const float* q_f32,
                         int64_t row_offset, int* flagged_out, float* flagged_thr_out, int flag_slot, int* ns_out,
                         cudaStream_t st) {
   int rc;
-  const int cap = (kprime <= 512) ? 1024 : 2048;
+  // reservoir size: the smallest that holds about k' more entries between two compactions
+  const int cap = reservoir_cap(kprime);
   // tier 2 keeps whatever the reservoir holds at the end (at most cap - 32 entries: a fuller one is compacted at once)
   const int out_cap = thr_init ? cap : kprime;
+  // candidates per query, all splits together: the rescore sorts them in shared memory (8 B each)
+  const int max_cands = (k <= 512) ? 4096 : kMaxCands;
   const int cg = ix->cta_group;
   const int clusters = (ix->max_ctas > 0 ? ix->max_ctas : gemm::sm_count()) / cg;
   const int q_tiles = static_cast<int>((nq + gemm::BM * cg - 1) / (gemm::BM * cg));
@@ -881,7 +1025,7 @@ int coarse_rescore_pass(ance_index* ix, const uint16_t* Q16, const float* q_f32,
     // split count whose work-item count fills whole waves best (ties: fewer splits = fewer candidates).
     n_splits = 1;
     if (q_tiles < 2 * clusters) {
-      const int max_splits = std::max(1, std::min(16, 4096 / out_cap));
+      const int max_splits = std::max(1, std::min(16, max_cands / out_cap));
       double best = -1.0;
       for (int sp = 1; sp <= max_splits; ++sp) {
         const long items = static_cast<long>(q_tiles) * sp;
@@ -891,17 +1035,22 @@ int coarse_rescore_pass(ance_index* ix, const uint16_t* Q16, const float* q_f32,
       }
     }
   }
-  while (n_splits > 1 && n_splits * out_cap > 4096) --n_splits;
-  ANCE_REQUIRE(n_splits * out_cap <= 4096, "ance_index_search: n_splits * candidates per split = %d exceeds 4096", n_splits * out_cap);
+  while (n_splits > 1 && n_splits * out_cap > max_cands) --n_splits;
+  ANCE_REQUIRE(n_splits * out_cap <= max_cands, "ance_index_search: n_splits * candidates per split = %d exceeds %d",
+               n_splits * out_cap, max_cands);
   int ns = 0;
   const bool bf = ix->fmt == ANCE_FMT_BF16;
 #define ANCE_COARSE(CG_, CAP_)                                                                                              \
   rc = bf ? launch_coarse<256, (CG_ == 1 ? 4 : 6), CG_, CAP_, tc05::kFmtBF16>(ix, Q16, nq, kprime, out_cap, thr_init, n_splits, &ns, st) \
           : launch_coarse<256, (CG_ == 1 ? 4 : 6), CG_, CAP_, tc05::kFmtF16>(ix, Q16, nq, kprime, out_cap, thr_init, n_splits, &ns, st)
   if (cg == 1 && cap == 1024) { ANCE_COARSE(1, 1024); }
-  else if (cg == 1) { ANCE_COARSE(1, 2048); }
+  else if (cg == 1 && cap == 2048) { ANCE_COARSE(1, 2048); }
+  else if (cg == 1 && cap == 4096) { ANCE_COARSE(1, 4096); }
+  else if (cg == 1) { ANCE_COARSE(1, 8192); }
   else if (cap == 1024) { ANCE_COARSE(2, 1024); }
-  else { ANCE_COARSE(2, 2048); }
+  else if (cap == 2048) { ANCE_COARSE(2, 2048); }
+  else if (cap == 4096) { ANCE_COARSE(2, 4096); }
+  else { ANCE_COARSE(2, 8192); }
 #undef ANCE_COARSE
   if (rc) return rc;
   *ns_out = ns;
@@ -1083,7 +1232,10 @@ extern "C" int ance_index_prepare(ance_index_t ix, void* stream) {
 extern "C" int ance_index_set_param(ance_index_t ix, const char* name, double value) {
   ANCE_REQUIRE(ix != nullptr && name != nullptr, "ance_index_set_param: null argument");
   const int v = static_cast<int>(value);
-  if (!strcmp(name, "kprime")) { ANCE_REQUIRE(v >= 0 && v <= 1024 && v % 32 == 0, "kprime must be a multiple of 32 in [0, 1024]"); ix->kprime = v; }
+  if (!strcmp(name, "kprime")) {
+    ANCE_REQUIRE(v >= 0 && v <= kMaxKprime && v % 32 == 0, "kprime must be a multiple of 32 in [0, %d]", kMaxKprime);
+    ix->kprime = v;
+  }
   else if (!strcmp(name, "n_splits")) { ANCE_REQUIRE(v >= 0 && v <= 64, "n_splits must be in [0, 64]"); ix->n_splits = v; }
   else if (!strcmp(name, "cta_group")) { ANCE_REQUIRE(v == 1 || v == 2, "cta_group must be 1 or 2"); ix->cta_group = v; }
   else if (!strcmp(name, "exact_fallback")) { ix->exact_fallback = v != 0; }
@@ -1108,7 +1260,8 @@ extern "C" int ance_index_set_param(ance_index_t ix, const char* name, double va
 extern "C" int ance_index_search_exact(ance_index_t ix, const float* q_dev, int64_t nq, int k, float* D_dev,
                                        int64_t* I_dev, int64_t row_offset, void* stream) {
   ANCE_REQUIRE(ix != nullptr, "ance_index_search_exact: null handle");
-  ANCE_REQUIRE(nq >= 0 && k > 0 && k <= 512, "ance_index_search_exact: need nq >= 0 and 0 < k <= 512");
+  ANCE_REQUIRE(nq >= 0 && k > 0, "ance_index_search_exact: need nq >= 0 and k > 0");
+  ANCE_REQUIRE(k <= kMaxK, "ance_index_search_exact: k = %d exceeds the largest supported k, %d", k, kMaxK);
   if (nq == 0) return ANCE_OK;
   ANCE_REQUIRE(q_dev && D_dev && I_dev, "ance_index_search_exact: null buffer");
   int rc = check_handle_device(ix, "ance_index_search_exact");
@@ -1131,6 +1284,7 @@ extern "C" int ance_index_search(ance_index_t ix, const float* q_dev, int64_t nq
   ANCE_REQUIRE(ix != nullptr, "ance_index_search: null handle");
   ANCE_REQUIRE(nq >= 0 && nq < (1ll << 31), "ance_index_search: nq out of range");
   ANCE_REQUIRE(k > 0, "ance_index_search: k must be positive");
+  ANCE_REQUIRE(k <= kMaxK, "ance_index_search: k = %d exceeds the largest supported k, %d", k, kMaxK);
   if (nq == 0) return ANCE_OK;
   ANCE_REQUIRE(q_dev && D_dev && I_dev, "ance_index_search: null buffer");
   int rc = check_handle_device(ix, "ance_index_search");
@@ -1139,14 +1293,17 @@ extern "C" int ance_index_search(ance_index_t ix, const float* q_dev, int64_t nq
   // choose k' (candidates kept per split).  The certificate needs every row within eps of the k-th score among the
   // candidates; eps is ~0.5 (fp16 operands) / ~3 (bf16) for rows of norm 27.7, i.e. ~0.1 k / ~0.6 k extra rows on the
   // distributions of tools/exp_certify.py.  A query that k' does not cover costs one tier-2 pass, not a wrong answer.
+  // k > 512 (up to kMaxK): the same formulas without the caps, served by the large reservoirs (reservoir_cap).
   int kprime = ix->kprime;
   if (kprime == 0) {
     const int want = (ix->fmt == ANCE_FMT_FP16) ? k + k / 2 - k / 16 : 2 * k + 32;   // fp16: ~1.44 k (k = 200: 288)
-    kprime = (k <= 240) ? std::min(512, std::max(64, (want + 31) / 32 * 32)) : std::min(992, (2 * k + 31) / 32 * 32);
+    if (k <= 240) kprime = std::min(512, std::max(64, (want + 31) / 32 * 32));
+    else if (k <= 512) kprime = std::min(992, (2 * k + 31) / 32 * 32);
+    else kprime = (want + 31) / 32 * 32;   // k = 1000: 1440 (fp16) / 2048 (bf16); k = 2048: 2944 / 4128
   }
-  if (kprime < k || kprime > 992 || k > 512 || ix->n < 4 * static_cast<int64_t>(kprime)) {
-    // tiny index or very large k: the exact brute-force path is both correct and cheap enough
-    ANCE_REQUIRE(k <= 512, "ance_index_search: k = %d > 512 is not supported", k);
+  const bool small_k = k <= 512;
+  if (kprime < k || (small_k && kprime > 992) || ix->n < 4 * static_cast<int64_t>(kprime)) {
+    // tiny index (or a k' set below k): the exact brute-force path is both correct and cheap enough
     ix->stats = ance_search_stats{};
     ix->stats.nq = nq;
     ix->stats.n_uncertified = nq;
@@ -1195,7 +1352,8 @@ extern "C" int ance_index_search(ance_index_t ix, const float* q_dev, int64_t nq
   }
   int n_exact = h[0];
   int ns2 = 0;
-  if (h[0] > 0 && ix->tier2 && ix->n >= 4 * 992) {
+  const int kprime2 = tier2_kprime(k);
+  if (h[0] > 0 && ix->tier2 && ix->n >= 4 * static_cast<int64_t>(kprime2)) {
     // --- tier 2: the uncertified queries once more, from their own thresholds (nothing that passes is dropped)
     const int n2 = h[0];
     if ((rc = ensure(&ix->Q16b, &ix->q16b_elems, static_cast<size_t>(n2) * ix->dim))) return rc;
@@ -1203,7 +1361,7 @@ extern "C" int ance_index_search(ance_index_t ix, const float* q_dev, int64_t nq
     gather_rows16_kernel<<<n2, 96, 0, st>>>(ix->Q16, ix->flagged, n2, ix->dim, ix->Q16b);
     ANCE_CUDA(cudaGetLastError());
     ance::count_launch(1);
-    rc = coarse_rescore_pass(ix, ix->Q16b, q_dev, n2, ix->flagged, 992, ix->flagged_thr, 0, k, D_dev, I_dev, row_offset,
+    rc = coarse_rescore_pass(ix, ix->Q16b, q_dev, n2, ix->flagged, kprime2, ix->flagged_thr, 0, k, D_dev, I_dev, row_offset,
                              ix->flagged2, nullptr, 3, &ns2, st);
     if (rc) return rc;
     ANCE_CUDA(cudaMemcpyAsync(h, ix->counters, sizeof(h), cudaMemcpyDeviceToHost, st));

@@ -35,6 +35,7 @@ import torch.distributed as dist
 from ..data import EmbeddingCache, StridedBatchReader
 from ..models import MSMarcoConfigDict
 from .. import postprocess
+from ..search import MAX_K
 
 logger = logging.getLogger(__name__)
 
@@ -366,6 +367,10 @@ def sharded_search_start(local_search: Callable, n_local_rows: int, queries_all:
     cuda = dev.type == "cuda"
     offset = int(row_offset) if row_offset is not None else int(sum(_shard_sizes(n_local_rows, dev)[:rank]))
     nq = int(queries_all.shape[0])
+    if k > 512:
+        # above k = 512 the block shrinks so that QB * k stays at most query_block * 512: the two pinned staging slots
+        # would otherwise grow with k (3.7 GB at k = 2048 and the default block)
+        query_block = max(1, query_block * 512 // k)
     QB = max(W, (max(1, min(query_block, nq)) + W - 1) // W * W)      # a multiple of W: equal all-to-all splits
     part = QB // W
     side = torch.cuda.Stream(device=dev) if cuda else None
@@ -549,6 +554,14 @@ def generate_new_ann(args, output_num, checkpoint_path, training_query_positive_
 # =============================================================================================
 # CLI (flags of run_ann_data_gen.py:443-627, plus three B200 knobs at the end)
 # =============================================================================================
+def topk_training_arg(value: str) -> int:
+    """argparse type of --topk_training: checked when the arguments are parsed, not after the corpus has been encoded."""
+    k = int(value)
+    if not 1 <= k <= MAX_K:
+        raise argparse.ArgumentTypeError("must be in [1, %d] (the largest k the search supports), got %d" % (MAX_K, k))
+    return k
+
+
 def get_arguments(argv=None):
     p = argparse.ArgumentParser()
     p.add_argument("--data_dir", default=None, type=str, required=True)
@@ -565,7 +578,8 @@ def get_arguments(argv=None):
     p.add_argument("--max_doc_character", default=10000, type=int)
     p.add_argument("--per_gpu_eval_batch_size", default=128, type=int)
     p.add_argument("--ann_chunk_factor", default=5, type=int)
-    p.add_argument("--topk_training", default=500, type=int)
+    p.add_argument("--topk_training", default=500, type=topk_training_arg,
+                   help="neighbours searched per training query, 1 .. %d" % MAX_K)
     p.add_argument("--negative_sample", default=5, type=int)
     p.add_argument("--ann_measure_topk_mrr", default=False, action="store_true")
     p.add_argument("--only_keep_latest_embedding_file", default=False, action="store_true")

@@ -186,7 +186,8 @@ def get_arguments(argv=None):
     p.add_argument("--max_doc_character", default=10000, type=int)
     p.add_argument("--per_gpu_eval_batch_size", default=128, type=int)
     p.add_argument("--ann_chunk_factor", default=5, type=int)
-    p.add_argument("--topk_training", default=500, type=int)
+    p.add_argument("--topk_training", default=500, type=base.topk_training_arg,
+                   help="neighbours searched per training query, 1 .. %d" % base.MAX_K)
     p.add_argument("--negative_sample", default=5, type=int)
     p.add_argument("--ann_measure_topk_mrr", default=False, action="store_true")
     p.add_argument("--only_keep_latest_embedding_file", default=False, action="store_true")

@@ -120,7 +120,8 @@ def eval_dev_query_full(query_embedding2id: np.ndarray, passage_embedding2id: np
 
 def full_rank(dev_query_embedding: np.ndarray, passage_embedding: np.ndarray, topN: int, device=None,
               block_rows: int = 1 << 20) -> np.ndarray:
-    """Notebook cell 13 on the GPU: exact top-N labels of every dev query over the whole (merged) passage matrix."""
+    """Notebook cell 13 on the GPU: exact top-N labels of every dev query over the whole (merged) passage matrix.
+    topN up to ance_b200.search.MAX_K (2048): the notebook's 1000 for MS MARCO passage runs as is."""
     import torch
     from .search import IndexFlatIP
     dev = device or torch.device("cuda", torch.cuda.current_device())
@@ -155,7 +156,8 @@ def rerank(dev_query_embedding: np.ndarray, dev_query_embedding2id: np.ndarray, 
 
 def evaluate_dumps(output_dir: str, step: int, dev_query_positive_id: Dict[int, Dict[int, int]], topN: int = 1000,
                    first_stage: Optional[Dict[int, Sequence[int]]] = None) -> Dict[str, Dict[str, float]]:
-    """Everything cells 9-13 print, from the dumps of `run_ann_data_gen --inference` at checkpoint `step`."""
+    """Everything cells 9-13 print, from the dumps of `run_ann_data_gen --inference` at checkpoint `step`.  The default
+    topN = 1000 is the notebook's full-rank depth for MS MARCO passage (Recall@1k); any topN <= 2048 is searched exactly."""
     q, q2id = load_dumps(output_dir, "dev_query_{}_".format(step))
     p, p2id = load_dumps(output_dir, "passage_{}_".format(step))
     res = {"full_rank": eval_dev_query_full(q2id, p2id, dev_query_positive_id, full_rank(q, p, min(topN, p.shape[0])), topN)}

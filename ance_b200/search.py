@@ -21,6 +21,9 @@ import torch
 
 from . import _lib
 
+#: largest k a search accepts (ance_index_search / ance_index_search_exact; faiss's GPU flat index has the same limit)
+MAX_K = 2048
+
 
 def _as_f32_cuda(x, device) -> torch.Tensor:
     if isinstance(x, np.ndarray):
@@ -132,7 +135,10 @@ class IndexFlatIP:
     # -- search ------------------------------------------------------------------------------------
     def search_device(self, q: torch.Tensor, k: int, row_offset: int = 0, exact: bool = False
                       ) -> Tuple[torch.Tensor, torch.Tensor]:
-        """Q [nq, d] fp32 CUDA -> (D [nq, k] fp32, I [nq, k] int64), both CUDA, stream-ordered."""
+        """Q [nq, d] fp32 CUDA -> (D [nq, k] fp32, I [nq, k] int64), both CUDA, stream-ordered.  1 <= k <= MAX_K."""
+        if int(k) > MAX_K:
+            # checked here too: an empty index or query batch never reaches the library, which refuses such a k
+            raise _lib.AnceError(f"k = {k} exceeds the largest supported k, {MAX_K}")
         nq = int(q.shape[0])
         D = torch.empty((nq, k), dtype=torch.float32, device=self.device)
         I = torch.empty((nq, k), dtype=torch.int64, device=self.device)

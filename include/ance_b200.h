@@ -44,6 +44,10 @@ int64_t ance_launch_count(void);
  * when fewer than k rows exist the tail is label -1 / score -FLT_MAX.  Ties are broken by the
  * smaller row number (faiss leaves tie order unspecified; ours is deterministic).
  * Scores are the exact fp32-input dot product accumulated in fp64 and rounded once to fp32.
+ * k is at most 2048 (faiss's GPU flat index has the same limit): ance_index_search and ance_index_search_exact fail with
+ * ANCE_ERR_INVALID and an error message naming the limit for k > 2048.  k <= 512 runs the register-resident coarse
+ * epilogue; 512 < k <= 2048 keeps larger candidate reservoirs in global memory (up to 1.2 GB of scratch on a 148-SM
+ * device, allocated the first time such a k is searched) and gives the same exact, certified results.
  * ance_index_search fails with ANCE_ERR_UNSUPPORTED when an index row or a query is non-finite after rounding to the
  * 16-bit operand format (inf / NaN input, or |x| > 65504 with ANCE_FMT_FP16) instead of returning unverifiable results.
  * ------------------------------------------------------------------------------------------------ */
@@ -84,7 +88,8 @@ int ance_index_search_exact(ance_index_t idx, const float* q_dev, int64_t nq, in
                             int64_t* I_dev, int64_t row_offset, void* stream);
 /* Statistics of the last search (ance_index_search has already synchronised its stream). */
 int ance_index_last_stats(ance_index_t idx, ance_search_stats* out);
-/* Tunables: "kprime" (0 = auto: about 1.44 k for fp16 operands, 2 k for bf16), "n_splits" (0 = auto), "cta_group" (1|2),
+/* Tunables: "kprime" (0 = auto: about 1.44 k for fp16 operands, 2 k for bf16; a multiple of 32 up to 4128 = 2 * 2048 + 32;
+ * a k' below k sends the search to the exact path), "n_splits" (0 = auto), "cta_group" (1|2),
  * "max_ctas" (0 = all SMs), "tier2" (0|1), "exact_fallback" (0|1: measurement only — results of uncertified queries are
  * then NOT guaranteed), "pace_window" (tiles a sweeping CTA pair may run ahead of the slowest one; 0 = no soft
  * barrier), "operand_fmt" (ANCE_FMT_*: the rows already added are re-rounded from the fp32 copy at the next prepare / search),
